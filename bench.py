@@ -1,10 +1,14 @@
 #!/usr/bin/env python
 """bench.py -- reads/sec of the alignment hot path (150 bp reads vs the 8 bundled rRNA databases).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--reads R] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--reads R] [--impl ours|reference] [--db-dir DIR] [--work-dir DIR]
+                  [--dump-outputs DIR]
 
-A "step" is one pass of the hot path over one batch of R synthetic reads per GPU (default: BASELINE.json
-config "10 M synthetic 150 bp Illumina reads vs all 8 data/rRNA_databases refs, 1xB200").
+A "step" is one pass of the hot path over one batch of R/K synthetic reads per GPU (default: BASELINE.json
+config "10 M synthetic 150 bp Illumina reads vs all 8 data/rRNA_databases refs, 1xB200").  The 8 databases are the FASTA
+files of --db-dir (the reference's data/rRNA_databases, e.g. as tools/stage_data.py stages them) or, by default, the seeded
+synthetic stand-ins of tools/synth_db.py; they and their index files live in a temporary directory for the run, or in
+--work-dir, where a later run finds and reuses them.
   value  : whole-job reads/s, kernels only, batch resident in HBM (CUDA events inside the C ABI)
   e2e    : reads/s through smr_align_batch with pinned HOST buffers (H2D + kernels + D2H inside the timed region)
   roofline: the seed-search kernel (dominant) against the measured HBM peak
@@ -15,6 +19,7 @@ import argparse
 import json
 import os
 import re
+import shutil
 import subprocess
 import sys
 import tempfile
@@ -27,11 +32,12 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 from sortmerna_b200 import hostio  # noqa: E402
-from tools import stage_data  # noqa: E402
+from tools import stage_data, synth_db  # noqa: E402
 
 READ_LEN = 150
 GEN_SEED = 20260924
 METRIC = "reads/sec (150 bp vs SILVA-8)"
+METRIC_SYNTHETIC = "reads/sec (150 bp vs synthetic SILVA-8)"
 
 
 # ------------------------------------------------------------------------------------------------
@@ -155,15 +161,19 @@ def write_fastq(path, reads):
 
 
 # ------------------------------------------------------------------------------------------------
-def load_databases(native_index=True):
-    stage_data.stage_inputs() if os.path.isdir(stage_data.REF_DATA) else None
-    fastas = [stage_data.db_path(n) for n in stage_data.DBS]
-    missing = [f for f in fastas if not os.path.exists(f)]
-    if missing:
-        raise SystemExit(f"missing database FASTA files {missing}: run tools/stage_data.py where /root/reference exists")
+def load_databases(tmp, db_dir=None, native_index=True):
+    """The 8 databases in --ref order: the FASTA files of db_dir, or the synthetic ones written under tmp; index files under tmp.
+    What tmp already holds is reused."""
+    if db_dir:
+        fastas = [os.path.join(db_dir, n + ".fasta") for n in stage_data.DBS]
+        missing = [f for f in fastas if not os.path.exists(f)]
+        if missing:
+            raise SystemExit(f"missing database FASTA files {missing}")
+    else:
+        fastas = synth_db.write_databases(os.path.join(tmp, "databases"))
     if not native_index:
         return fastas, None, None, [hostio.load_references(f) for f in fastas], None, {}
-    idx_dir, built = stage_data.ensure_indexes(fastas)   # smr_build_index (our builder), 8 databases in parallel
+    idx_dir, built = stage_data.ensure_indexes(fastas, os.path.join(tmp, "idx"))   # smr_build_index (our builder), 8 databases in parallel
     pre = hostio.find_index_prefixes(idx_dir)
     refs = [hostio.load_references(f) for f in fastas]
     stats = [hostio.parse_stats(pre[os.path.basename(f)]) for f in fastas]
@@ -199,10 +209,18 @@ def survey_8d_seed(fastas, prefixes, refs, ms, stats, reads03, threads, reads_pe
             "sample": f"oracle walk (reference pass schedule + pruned DFS) on the first {n} reads of the workload, 8 databases"}
 
 
-def reference_index_dir(fastas):
+def db_source(args):
+    return os.path.abspath(args.db_dir) if args.db_dir else f"synthetic (tools/synth_db.py, seed {synth_db.SEED})"
+
+
+def db_words(args):
+    return "all 8 data/rRNA_databases refs" if args.db_dir else "synthetic stand-ins of the 8 data/rRNA_databases refs"
+
+
+def reference_index_dir(fastas, tmp):
     """The reference legs (cpu_baseline, --impl reference) run the unmodified binary on the index ITS OWN builder makes
-    (data_cache/idx_ref; one process per database, outside every timed region) -- never on files our builder wrote."""
-    d, _ = stage_data.ensure_indexes(fastas, os.path.join(stage_data.CACHE, "idx_ref"), builder="reference")
+    (<tmp>/idx_ref; one process per database, outside every timed region) -- never on files our builder wrote."""
+    d, _ = stage_data.ensure_indexes(fastas, os.path.join(tmp, "idx_ref"), builder="reference")
     return d
 
 
@@ -288,15 +306,15 @@ def host_cores():
     return eff, dict(os_cpu_count=ncpu, affinity=aff, cgroup_quota=quota, threads_used=eff, loadavg_1m=load)
 
 
-def cli_e2e(args, cores, core_info):
+def cli_e2e(args, cores, core_info, tmp):
     """What a user runs: the reference's host program with the binding (oracle/_ref/sortmerna_gpu -ref x8 -reads file.fq) against
     the unmodified reference binary on the same file -- 'Done alignment' seconds and total wall, flat FASTQ (and .gz with
     --cli-gz).  The CPU binary gets a bounded prefix of the same file (its cost is linear in reads)."""
     import gzip
     import shutil
     from oracle import ora
-    fastas, idx_dir, _, refs, _, _ = load_databases()
-    ref_idx = reference_index_dir(fastas)
+    fastas, idx_dir, _, refs, _, _ = load_databases(tmp, args.db_dir)
+    ref_idx = reference_index_dir(fastas, tmp)
     pool = DbPool(refs)
     n = args.cli_reads
     gpu_bin = os.path.join(ROOT, "oracle", "_ref", "sortmerna_gpu")
@@ -346,6 +364,38 @@ INSTR_ONLY = ("windows", "trie_nodes", "buckets", "bucket_entries", "dbg_max_rea
               "dbg_max_read_busy_cycles")
 
 
+# the per-read and per-alignment fields --dump-outputs writes (cigar_off is a position in the batch's CIGAR pool: the words
+# themselves are written instead), and the counters that count algorithmic work (the same in every run of the same inputs)
+DUMP_RES_FIELDS = ["lastIndex", "lastPart", "hit_seeds", "min_index", "max_index", "n_align", "max_SW_count", "is_done", "is_hit"]
+DUMP_ALN_FIELDS = ["cigar_len", "ref_num", "ref_begin1", "ref_end1", "read_begin1", "read_end1", "readlen", "score1", "part", "index_num", "strand"]
+DUMP_COUNTERS = ("num_aligned", "sw_calls", "sw_cells", "pos_entries", "lis_calls")
+DUMP_READS = 1 << 16
+
+
+def dump_outputs(out_dir, res, read0):
+    """What the last timed step returned to its caller (api.Aligner.download()), as float64 .npy files: every field of
+    the per-read results and of the stored alignments of a fixed, seeded sample of DUMP_READS reads, their CIGAR words,
+    the per-database match counts and the algorithmic counters of the whole batch.  read0: global number of the batch's
+    first read."""
+    os.makedirs(out_dir, exist_ok=True)
+    n, slots = res["res"].shape[0], int(res["slots"])
+    pick = np.sort(np.random.default_rng(GEN_SEED).choice(n, min(n, DUMP_READS), replace=False))
+    arrays = {"read_index": pick + read0}
+    for f in DUMP_RES_FIELDS:
+        arrays["res." + f] = res["res"][f][pick]
+    alns = res["alns"].reshape(n, slots)[pick] if slots else res["alns"][:0]
+    for f in DUMP_ALN_FIELDS:
+        arrays["alns." + f] = alns[f]
+    flat = alns.reshape(-1)
+    cig = res["cigar"]
+    arrays["cigar"] = np.concatenate([cig[int(o):int(o) + int(k)] for o, k in zip(flat["cigar_off"], flat["cigar_len"])] or [cig[:0]])
+    arrays["matched"] = res["matched"]
+    for k in DUMP_COUNTERS:
+        arrays["counters." + k] = np.array([res["counters"][k]])
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -371,7 +421,22 @@ def main():
     ap.add_argument("--cli-cpu-reads", type=int, default=100_000)
     ap.add_argument("--cli-gpus", type=int, default=1)
     ap.add_argument("--cli-gz", action="store_true")
+    ap.add_argument("--db-dir", default=None, help="directory of the 8 database FASTA files (default: the synthetic databases of tools/synth_db.py)")
+    ap.add_argument("--work-dir", default=None, help="where the databases and their index files are written, and reused by later runs "
+                                                     "(default: a temporary directory of this run)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step returned (a seeded sample of the reads, every result field) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    tmp = tempfile.mkdtemp(prefix="smr_bench_")     # databases, index files, reference work directories: never in the tree
+    try:
+        run(args, tmp)
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)
+
+
+def run(args, tmp):
     # stdout carries exactly ONE JSON line: everything else that writes to fd 1 (NCCL's version banner, library chatter) goes to stderr
     sys.stdout.flush()
     json_fd = os.dup(1)
@@ -385,15 +450,16 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     cores, core_info = host_cores()
 
+    work = args.work_dir or tmp
     if args.cli_e2e:
-        emit({"cli_e2e": cli_e2e(args, cores, core_info)})
+        emit({"cli_e2e": cli_e2e(args, cores, core_info, work)})
         return
 
     if args.impl == "reference":
         if rank != 0:
             return
-        fastas, _, _, refs, _, _ = load_databases(native_index=False)
-        idx_dir = reference_index_dir(fastas)
+        fastas, _, _, refs, _, _ = load_databases(work, args.db_dir, native_index=False)
+        idx_dir = reference_index_dir(fastas, work)
         pool = DbPool(refs)
         # ~10 s of reference CPU time per step (about 230 reads/s per core on this workload): large enough that thread start-up
         # and the skew between the reference's static per-thread splits do not dominate (round 1: 300 reads per thread did)
@@ -409,12 +475,12 @@ def main():
         v = float(np.mean(vals))
         desc = f"{sample} synthetic 150 bp reads per step vs the 8 databases, alignment loops only (index loading excluded), -threads {cores}"
         emit(({
-            "metric": METRIC, "value": v, "unit": "reads/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
+            "metric": METRIC if args.db_dir else METRIC_SYNTHETIC, "value": v, "unit": "reads/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": 1000.0 * float(np.mean(secs)), "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "int16/u8 (SSE2)", "data": "synthetic", "impl": "reference",
-            "config": {"workload": "10 M synthetic 150 bp Illumina reads vs all 8 data/rRNA_databases refs, 1xB200",
+            "config": {"workload": f"10 M synthetic 150 bp Illumina reads vs {db_words(args)}, 1xB200",
                        "sampled": "each step is a bounded sample of that workload (reads_per_step reads, same generator)",
-                       "reads_per_step": sample, "read_len": READ_LEN, "databases": 8},
+                       "reads_per_step": sample, "read_len": READ_LEN, "databases": 8, "database_files": db_source(args)},
             "cpu_baseline": {"value": v, "unit": "reads/s", "cores": cores, "kind": "reference", "sample": desc, "host": core_info,
                              "per_step": [float(x) for x in vals]},
             "e2e": {"value": v, "unit": "reads/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -428,11 +494,14 @@ def main():
         torch.cuda.set_device(local_rank)
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     t_setup = time.time()
-    if world > 1:       # the index cache is built once (rank 0), the other ranks wait and then only read it
+    if world > 1:       # the databases and their indexes are made once (rank 0, in its directory), the other ranks wait and then only read them
+        shared = [work]
+        dist.broadcast_object_list(shared, src=0)
+        work = shared[0]
         if rank == 0:
-            load_databases()
+            load_databases(work, args.db_dir)
         dist.barrier()
-    fastas, idx_dir, prefixes, refs, stats, built = load_databases()
+    fastas, idx_dir, prefixes, refs, stats, built = load_databases(work, args.db_dir)
     n_job = args.reads
     n = max(1, n_job // args.steps)                   # reads per step (batch) per GPU
     ms = minimal_scores(stats, fastas, n_job * world)  # refstats totals stay GLOBAL across shards (SURVEY 8(e))
@@ -483,6 +552,7 @@ def main():
         vec_s = np.array([res["counters"][k] for k in api.CNT_NAMES] + [int(x) for x in res["matched"]], dtype=np.int64)
         csum = vec_s if csum is None else csum + vec_s
     barrier()
+    last_res = res
     wall_ms = (time.perf_counter() - t0) * 1000.0
     sampler.stop_flag = True; sampler.join(timeout=2)
     step_ms = float(np.sum(dev_ms))          # CUDA events on the library's stream, summed over the K steps
@@ -596,12 +666,13 @@ def main():
                  "peak_source": peak_src, "algorithmic_bytes_per_step": int(alg_bytes / world / args.steps),
                  "kernel_ms_per_step": float(np.mean(seed_ms))}
     out = {
-        "metric": METRIC, "value": value, "unit": "reads/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
+        "metric": METRIC if args.db_dir else METRIC_SYNTHETIC, "value": value, "unit": "reads/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
         "ms_per_step": tm[0] / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "int16x2 (DPX) / u8", "data": "synthetic",
-        "config": {"workload": "10 M synthetic 150 bp Illumina reads vs all 8 data/rRNA_databases refs, 1xB200" if (n_job == 10_000_000 and world == 1) else
-                   f"{n_job} synthetic 150 bp Illumina reads per GPU vs all 8 data/rRNA_databases refs",
-                   "reads_per_gpu_per_step": n, "reads_per_gpu_job": n * args.steps, "read_len": READ_LEN, "databases": 8, "index_hbm_bytes": info["hbm_bytes"],
+        "config": {"workload": f"10 M synthetic 150 bp Illumina reads vs {db_words(args)}, 1xB200" if (n_job == 10_000_000 and world == 1) else
+                   f"{n_job} synthetic 150 bp Illumina reads per GPU vs {db_words(args)}",
+                   "reads_per_gpu_per_step": n, "reads_per_gpu_job": n * args.steps, "read_len": READ_LEN, "databases": 8,
+                   "database_files": db_source(args), "index_hbm_bytes": info["hbm_bytes"],
                    "l2": "inputs larger than L2 (index 1.3 GB + reads 1.5 GB per pass)", "parallelism": f"reads sharded by record x{world}",
                    "hit_rate": counters["num_aligned"] / total_reads_job},
         "e2e": {"value": e2e_value, "unit": "reads/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h},
@@ -617,9 +688,13 @@ def main():
         "counters": counters,
         "setup_s": setup_s, "index_build_s": built, "index_source": args.index_source, "index_resident_s": round(index_resident_s, 2),
     }
-    if not args.no_cpu_baseline and world == 1:   # reported baseline: rank 0 at N = 1 only
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_res, (args.steps - 1) * n)
+    if not args.no_cpu_baseline and world == 1 and not os.path.exists(stage_data.REF_BIN):
+        out["cpu_baseline"] = {"unavailable": "the reference CPU build (oracle/_ref/sortmerna_ref) is not built"}
+    elif not args.no_cpu_baseline and world == 1:   # reported baseline: rank 0 at N = 1 only
         sample = min(n, args.cpu_sample or int(min(400_000, max(20_000, 2_300 * cores))))
-        v, t, total, _ = run_reference_sample(fastas, reference_index_dir(fastas), first_reads[:sample], cores)
+        v, t, total, _ = run_reference_sample(fastas, reference_index_dir(fastas, work), first_reads[:sample], cores)
         out["cpu_baseline"] = {"value": v, "unit": "reads/s", "cores": cores, "kind": "reference", "host": core_info,
                                "sample": f"first {sample} reads of the same synthetic workload vs the 8 databases, reference CPU build "
                                          f"(oracle/_ref/sortmerna_ref -threads {cores}), alignment loops {t:.1f} s (index loading excluded; "

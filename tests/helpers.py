@@ -1,5 +1,37 @@
 """Shared helpers of the parity tests."""
+import gzip
+import os
+
 import numpy as np
+
+SETS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "sets")
+# the parity samples of the bundled read sets: the first 100 records of set2 and of both set4 mates (tests/golden/make_sets.py)
+SET2_SAMPLE = os.path.join(SETS, "set2_environmental_study_550_amplicon.head100.fasta.gz")
+SET4_SAMPLES = [os.path.join(SETS, f"set4_mate_pairs_metatranscriptomics_{k}.head100.fastq.gz") for k in (1, 2)]
+ID85 = "silva-bac-16s-database-id85"
+
+
+def stored_databases(workdir, names):
+    """tests/golden/sets/<name>.hits.fasta.gz (the sequences of a bundled database the parity samples align to and its first
+    three, made by tests/golden/make_sets.py) unpacked as <workdir>/<name>.fasta; returns the paths in the order of names"""
+    out = []
+    for n in names:
+        p = os.path.join(workdir, n + ".fasta")
+        with open(p, "wb") as f:
+            f.write(gzip.decompress(open(os.path.join(SETS, n + ".hits.fasta.gz"), "rb").read()))
+        out.append(p)
+    return out
+
+
+def unpacked(workdir, gz_paths):
+    """the stored .gz read samples unpacked into workdir; returns the paths"""
+    out = []
+    for g in gz_paths:
+        p = os.path.join(workdir, os.path.basename(g)[:-3])
+        with open(p, "wb") as f:
+            f.write(gzip.decompress(open(g, "rb").read()))
+        out.append(p)
+    return out
 
 
 def params_kwargs_from_args(args):

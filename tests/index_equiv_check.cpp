@@ -6,6 +6,9 @@
 //   .pos       same N; list of id a == list of id b (same order) under that bijection
 //   .stats     identical apart from the embedded FASTA path and the 4 padding bytes of each index_parts_stats record
 // Usage: index_equiv_check <prefixA> <prefixB> <lnwin>.  Prints "OK ..." and exits 0, or the first difference and exits 1.
+//        index_equiv_check --canonical <prefix> <lnwin> <out>: writes a form of the index that equivalent indexes share (the
+//        .stats FASTA size and body without path and padding, then per part the .kmer bytes, the .bursttrie with every id replaced by its
+//        rank of first appearance, and the position lists in that order), so that a digest of it stands for the index.
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -44,7 +47,70 @@ static Stats parse_stats(const std::string& p) {
   return s;
 }
 
+static int canonical(const std::string& A, uint32_t lnwin, const std::string& out_path) {
+  const uint32_t limit = 1u << lnwin;
+  const Stats sa = parse_stats(A + ".stats");
+  std::vector<uint8_t> out((const uint8_t*)&sa.fsize, (const uint8_t*)&sa.fsize + 8);
+  auto put = [&](const uint8_t* p, size_t n) { out.insert(out.end(), p, p + n); };
+  put(sa.rest_wo_pad.data(), sa.rest_wo_pad.size());
+  auto put32 = [&](uint32_t x) { put((const uint8_t*)&x, 4); };
+  for (uint16_t part = 0; part < sa.parts; ++part) {
+    const std::string ps = std::to_string(part);
+    bool ok;
+    auto ka = slurp(A + ".kmer_" + ps + ".dat", ok);
+    if (!ok) die("kmer file missing");
+    auto ta = slurp(A + ".bursttrie_" + ps + ".dat", ok);
+    if (!ok) die("bursttrie file missing");
+    auto pa = slurp(A + ".pos_" + ps + ".dat", ok);
+    if (!ok) die("pos file missing");
+    put(ka.data(), ka.size());
+    const uint32_t N = u32(pa, 0);
+    std::vector<uint32_t> rank(N, 0xFFFFFFFFu), order;
+    size_t o = 0;
+    for (uint32_t i = 0; i < limit; ++i) {
+      const uint32_t sz[2] = {u32(ta, o), u32(ta, o + 4)};
+      put(&ta[o], 8);
+      o += 8;
+      for (int j = 0; j < 2; ++j) {
+        if (!sz[j]) continue;
+        std::deque<uint8_t> fifo;
+        for (int k = 0; k < 4; ++k) { fifo.push_back(ta[o]); put(&ta[o], 1); ++o; }
+        while (!fifo.empty()) {
+          const uint8_t f = fifo.front(); fifo.pop_front();
+          if (f == 1) { for (int k = 0; k < 4; ++k) { fifo.push_back(ta[o]); put(&ta[o], 1); ++o; } }
+          else if (f == 2) {
+            const uint32_t bytes = u32(ta, o);
+            put(&ta[o], 4);
+            o += 4;
+            for (uint32_t e = 0; e < bytes / 8; ++e, o += 8) {
+              const uint32_t id = u32(ta, o + 4);
+              if (id >= N) die("id out of range");
+              if (rank[id] == 0xFFFFFFFFu) { rank[id] = (uint32_t)order.size(); order.push_back(id); }
+              put(&ta[o], 4);
+              put32(rank[id]);
+            }
+          } else if (f != 0) die("bad flag");
+        }
+      }
+    }
+    if (o != ta.size()) die("trailing bytes in bursttrie");
+    if (order.size() != N) die("an id never appears in a bucket");
+    std::vector<size_t> offa(N);
+    size_t oa = 4;
+    for (uint32_t i = 0; i < N; ++i) { offa[i] = oa; oa += 4 + (size_t)u32(pa, oa) * 8; }
+    if (oa != pa.size()) die("pos file length");
+    put32(N);
+    for (uint32_t id : order) put(&pa[offa[id]], 4 + (size_t)u32(pa, offa[id]) * 8);
+  }
+  FILE* f = fopen(out_path.c_str(), "wb");
+  if (!f || fwrite(out.data(), 1, out.size(), f) != out.size()) die("cannot write " + out_path);
+  fclose(f);
+  printf("OK parts=%u bytes=%zu\n", sa.parts, out.size());
+  return 0;
+}
+
 int main(int argc, char** argv) {
+  if (argc == 5 && std::string(argv[1]) == "--canonical") return canonical(argv[2], (uint32_t)atoi(argv[3]), argv[4]);
   if (argc < 4) { fprintf(stderr, "usage: %s prefixA prefixB lnwin\n", argv[0]); return 2; }
   const std::string A = argv[1], B = argv[2];
   const uint32_t lnwin = (uint32_t)atoi(argv[3]), limit = 1u << lnwin;

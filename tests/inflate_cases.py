@@ -49,12 +49,34 @@ def cases(n_reads: int = 6000):
     with gzip.GzipFile(filename="reads_file.fq", mode="wb", fileobj=bio, mtime=123) as g:
         g.write(txt[:70000])
     out.append(("header_fname", bio.getvalue(), txt[:70000]))
-    for fn in ("set4_mate_pairs_metatranscriptomics_1.fastq.gz", "set4_mate_pairs_metatranscriptomics_2.fastq.gz"):
-        p = os.path.join(ROOT, "data_cache", "sets", fn)
-        if os.path.exists(p):
-            raw = open(p, "rb").read()
-            out.append((fn[:28], raw, gzip.decompress(raw)))
+    sampled = rrna_fastq_text(12000)
+    out.append(("rrna_reads", gzip.compress(sampled, 6), sampled))
+    raw = open(SET4_HEAD, "rb").read()
+    out.append(("set4_head", raw, gzip.decompress(raw)))
     return out
+
+
+SET4_HEAD = os.path.join(ROOT, "tests", "golden", "sets", "set4_mate_pairs_metatranscriptomics_1.head500.fastq.gz")
+
+
+def rrna_fastq_text(n: int, seed: int = 11) -> bytes:
+    """Reads of 100 nt cut from the golden rRNA slices with 1 % substitutions, Illumina-like headers and qualities: text that
+    compresses like a real read file (long deflate streams of many blocks), made in memory."""
+    rng = np.random.default_rng(seed)
+    seqs = []
+    for g in ("db_arc.fasta", "db_bac.fasta"):
+        with open(os.path.join(ROOT, "tests", "golden", g), "rb") as f:
+            seqs += [b"".join(rec.split(b"\n")[1:]) for rec in f.read().split(b">")[1:]]
+    out = []
+    for i in range(n):
+        s = seqs[int(rng.integers(0, len(seqs)))]
+        b = int(rng.integers(0, len(s) - 100))
+        r = bytearray(s[b:b + 100])
+        for k in np.flatnonzero(rng.random(100) < 0.01):
+            r[k] = b"ACGT"[int(rng.integers(0, 4))]
+        q = bytes((rng.integers(28, 41, 100) + 33 - (np.arange(100) > 80) * rng.integers(0, 20, 100)).astype(np.uint8))
+        out.append(b"@sample.%09d/1 length=100 begin=%d\n%s\n+\n%s\n" % (i, b, bytes(r), q))
+    return b"".join(out)
 
 
 def bad_cases():

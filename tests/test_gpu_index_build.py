@@ -103,12 +103,11 @@ def test_device_index_equals_host_builder_with_options(golden, name, kw):
 
 
 def test_device_index_bundled_database_and_time():
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    fasta = os.path.join(root, "data_cache", "rRNA_databases", "silva-arc-16s-id95.fasta")
-    if not os.path.exists(fasta):
-        pytest.skip("data_cache not staged")
+    """A database of the size of silva-arc-16s-id95 (tools/synth_db.py's stand-in: 3193 sequences of ~1.1 kb)."""
     import time
+    from tools import synth_db
     with tempfile.TemporaryDirectory(prefix="smr_devidx_") as d:
+        fasta = synth_db.write_databases(d, only=["silva-arc-16s-id95"])[0]
         prefix = os.path.join(d, "arc16s")
         t0 = time.time(); api.build_index(fasta, prefix); t_host = time.time() - t0
         refs = hostio.load_references(fasta)

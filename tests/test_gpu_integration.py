@@ -1,5 +1,8 @@
 """The drop-in, end to end on the GPU: the unmodified reference host program linked with integration/align_gpu.cpp and the
-PRODUCT library (oracle/_ref/sortmerna_gpu) writes the files the reference binary writes for the same command line."""
+PRODUCT library (oracle/_ref/sortmerna_gpu) writes the files the reference binary writes for the same command line.
+The bundled-set cases run on stored samples (tests/golden/sets/: the first 100 records of both set4 mates and the sequences of
+the databases they align to); where data_cache/ holds the full bundled data (tools/stage_data.py) they also run at full size,
+with the known answers of scripts/test.jinja."""
 import os
 import shutil
 import tempfile
@@ -7,6 +10,7 @@ import tempfile
 import pytest
 
 from conftest import GOLDEN
+from helpers import ID85, SET4_SAMPLES, stored_databases, unpacked
 from integration_common import REF_DIR, assert_same_outputs, run_host
 
 pytestmark = pytest.mark.gpu
@@ -37,35 +41,52 @@ def test_reference_t9_golden_sam_rows_on_gpu():
     assert run_t9("sortmerna_gpu") == T9_ROWS
 
 
+def _need_binaries():
+    for b in ("sortmerna_ref", "sortmerna_gpu"):
+        if not os.path.exists(os.path.join(REF_DIR, b)):
+            pytest.skip(f"oracle/_ref/{b} not built (oracle/Makefile.ref)")
+
+
 def test_reference_t5_mate_pairs_known_answer():
-    """scripts/test.jinja t5: the two set4 mate files (2 x 5000 reads, paired feed, 5 threads) vs silva-bac-16s-id85 built with
-    -max_pos 250: 10000 reads -> 6000 aligned / 4000 not; the drop-in host program on the GPU against the reference binary."""
-    import subprocess
+    """scripts/test.jinja t5: the two set4 mate files (paired feed, 5 threads) vs silva-bac-16s-id85 built with -max_pos 250; the
+    drop-in host program on the GPU against the reference binary.  Stored sample: 2 x 100 mates vs the sequences of the database
+    they align to; at full size 2 x 5000 mates vs the whole database: 10000 reads -> 6000 aligned / 4000 not."""
     from conftest import ROOT
     from tools import stage_data
-    cache = os.path.join(ROOT, "data_cache")
-    fasta = os.path.join(cache, "sets", "silva-bac-16s-database-id85.fasta")
-    reads = [os.path.join(cache, "sets", f"set4_mate_pairs_metatranscriptomics_{k}.fastq") for k in (1, 2)]
-    for p in [fasta] + reads + [os.path.join(REF_DIR, "sortmerna_gpu"), os.path.join(REF_DIR, "sortmerna_ref")]:
-        if not os.path.exists(p):
-            pytest.skip(f"{p} missing")
-    idx, _ = stage_data.ensure_indexes([fasta], os.path.join(cache, "idx_set2_ref"), extra=("-max_pos", "250"), builder="reference")
+    _need_binaries()
     d = tempfile.mkdtemp(prefix="smr_t5_")
     try:
-        outs = {}
-        for b in ("sortmerna_ref", "sortmerna_gpu"):
-            wd = os.path.join(d, b)
-            cmd = [os.path.join(REF_DIR, b), "-ref", fasta, "-reads", reads[0], "-reads", reads[1], "-max_pos", "250", "-fastx", "-other", "-threads", "5",
-                   "-workdir", wd, "-idx-dir", idx, "-task", "4"]
-            p = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=900)
-            assert p.returncode == 0, p.stdout[-2000:]
-            log = open(os.path.join(wd, "out", "aligned.log")).read()
-            outs[b] = (log, {fn: open(os.path.join(wd, "out", fn)).read() for fn in os.listdir(os.path.join(wd, "out")) if fn.endswith(".fq")})
-        for b in outs:
-            assert "passing E-value threshold = 6000" in outs[b][0] and "failing E-value threshold = 4000" in outs[b][0], b   # scripts/test.jinja:318-322
-        assert outs["sortmerna_gpu"][1] == outs["sortmerna_ref"][1]
+        fasta = stored_databases(d, [ID85])[0]
+        idx, _ = stage_data.ensure_indexes([fasta], os.path.join(d, "idx_ref"), extra=("-max_pos", "250"), builder="reference")
+        _t5(fasta, unpacked(d, SET4_SAMPLES), idx, os.path.join(d, "sample"), None)
+        cache = os.path.join(ROOT, "data_cache")
+        fasta = os.path.join(cache, "sets", "silva-bac-16s-database-id85.fasta")
+        reads = [os.path.join(cache, "sets", f"set4_mate_pairs_metatranscriptomics_{k}.fastq") for k in (1, 2)]
+        if all(os.path.exists(p) for p in [fasta] + reads):
+            idx, _ = stage_data.ensure_indexes([fasta], os.path.join(cache, "idx_set2_ref"), extra=("-max_pos", "250"), builder="reference")
+            _t5(fasta, reads, idx, os.path.join(d, "full"), (6000, 4000))      # scripts/test.jinja:318-322
     finally:
         shutil.rmtree(d, ignore_errors=True)
+
+
+def _t5(fasta, reads, idx, d, known):
+    import subprocess
+    outs = {}
+    for b in ("sortmerna_ref", "sortmerna_gpu"):
+        wd = os.path.join(d, b)
+        cmd = [os.path.join(REF_DIR, b), "-ref", fasta, "-reads", reads[0], "-reads", reads[1], "-max_pos", "250", "-fastx", "-other", "-threads", "5",
+               "-workdir", wd, "-idx-dir", idx, "-task", "4"]
+        p = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=900)
+        assert p.returncode == 0, p.stdout[-2000:]
+        log = open(os.path.join(wd, "out", "aligned.log")).read()
+        outs[b] = ([ln for ln in log.split("\n") if "E-value threshold" in ln],
+                   {fn: open(os.path.join(wd, "out", fn)).read() for fn in os.listdir(os.path.join(wd, "out")) if fn.endswith(".fq")})
+    assert outs["sortmerna_gpu"][0] == outs["sortmerna_ref"][0]
+    if known:
+        for b in outs:
+            log = "\n".join(outs[b][0])
+            assert f"passing E-value threshold = {known[0]}" in log and f"failing E-value threshold = {known[1]}" in log, b
+    assert outs["sortmerna_gpu"][1] == outs["sortmerna_ref"][1]
 
 
 def _run_binary(binary, fastas, reads, idx, wd, extra, threads=8, env=None):
@@ -90,55 +111,76 @@ def _run_binary(binary, fastas, reads, idx, wd, extra, threads=8, env=None):
     return files, p.stdout
 
 
-def _config4_inputs():
+def _config4_sample(d):
+    """The stored sample of BASELINE config 4: both set4 mates (2 x 100 reads, FASTQ.gz as stored) vs the sequences of the 8
+    rRNA databases they align to -- (databases, reads, the reference builder's index)"""
+    from tools import stage_data
+    fastas = stored_databases(d, stage_data.DBS)
+    idx, _ = stage_data.ensure_indexes(fastas, os.path.join(d, "idx_ref"), builder="reference")
+    return fastas, list(SET4_SAMPLES), idx
+
+
+def _config4_full():
+    """BASELINE config 4 at full size where data_cache/ holds it, else None"""
     from conftest import ROOT
     from tools import stage_data
     cache = os.path.join(ROOT, "data_cache")
     reads = [os.path.join(cache, "sets", f"set4_mate_pairs_metatranscriptomics_{k}.fastq.gz") for k in (1, 2)]
     fastas = [stage_data.db_path(n) for n in stage_data.DBS]
-    for p in reads + fastas + [os.path.join(REF_DIR, "sortmerna_gpu"), os.path.join(REF_DIR, "sortmerna_ref")]:
-        if not os.path.exists(p):
-            pytest.skip(f"{p} missing")
+    if not all(os.path.exists(p) for p in reads + fastas):
+        return None
     idx, _ = stage_data.ensure_indexes(fastas, os.path.join(cache, "idx_ref"), builder="reference")
     return fastas, reads, idx
 
 
 def test_baseline_config4_through_the_binary():
-    """BASELINE config 4 as written: set4 paired FASTQ.gz vs the 8 rRNA databases, -sam, through the CLI of the drop-in host program
-    (gz inflate + paired feed + 8 resident indexes + report stage) against the unmodified reference binary: 5944 / 4056
-    (scripts/test.jinja t17) and identical SAM rows / aligned / other reads."""
-    fastas, reads, idx = _config4_inputs()
+    """BASELINE config 4: set4 paired FASTQ.gz vs the 8 rRNA databases, -sam, through the CLI of the drop-in host program
+    (gz inflate + paired feed + 8 resident indexes + report stage) against the unmodified reference binary: identical SAM rows /
+    aligned / other reads, with the indexes read from the files and built on the GPU.  Stored sample always; at full size also
+    the known answer 5944 / 4056 (scripts/test.jinja t17)."""
+    _need_binaries()
     d = tempfile.mkdtemp(prefix="smr_cfg4_")
     try:
-        extra = ["-sam", "-fastx", "-other", "-paired_in"]
-        ref, _ = _run_binary("sortmerna_ref", fastas, reads, idx, os.path.join(d, "ref"), extra)
-        got, log = _run_binary("sortmerna_gpu", fastas, reads, idx, os.path.join(d, "got"), extra)
-        assert "Starting alignment (libsmr_b200)" in log
-        assert any("passing E-value threshold = 5944" in ln for ln in got["aligned.log"]) and any("failing E-value threshold = 4056" in ln for ln in got["aligned.log"])
-        assert sorted(got) == sorted(ref)
-        for fn in got:
-            assert got[fn] == ref[fn], fn
-        # the same with the 8 indexes built on the GPU from the FASTA files (smr_build_index_device) instead of read from the index files
-        dev, log = _run_binary("sortmerna_gpu", fastas, reads, idx, os.path.join(d, "dev"), extra, env=dict(os.environ, SMR_INDEX_DEVICE="1"))
-        assert "Starting alignment (libsmr_b200)" in log
-        for fn in ref:
-            assert dev[fn] == ref[fn], "device-built index: " + fn
+        _config4(*_config4_sample(d), os.path.join(d, "sample"), None)
+        full = _config4_full()
+        if full:
+            _config4(*full, os.path.join(d, "full"), (5944, 4056))
     finally:
         shutil.rmtree(d, ignore_errors=True)
 
 
+def _config4(fastas, reads, idx, d, known):
+    extra = ["-sam", "-fastx", "-other", "-paired_in"]
+    ref, _ = _run_binary("sortmerna_ref", fastas, reads, idx, os.path.join(d, "ref"), extra)
+    got, log = _run_binary("sortmerna_gpu", fastas, reads, idx, os.path.join(d, "got"), extra)
+    assert "Starting alignment (libsmr_b200)" in log
+    if known:
+        assert any(f"passing E-value threshold = {known[0]}" in ln for ln in got["aligned.log"])
+        assert any(f"failing E-value threshold = {known[1]}" in ln for ln in got["aligned.log"])
+    assert sorted(got) == sorted(ref)
+    for fn in got:
+        assert got[fn] == ref[fn], fn
+    # the same with the 8 indexes built on the GPU from the FASTA files (smr_build_index_device) instead of read from the index files
+    dev, log = _run_binary("sortmerna_gpu", fastas, reads, idx, os.path.join(d, "dev"), extra, env=dict(os.environ, SMR_INDEX_DEVICE="1"))
+    assert "Starting alignment (libsmr_b200)" in log
+    for fn in ref:
+        assert dev[fn] == ref[fn], "device-built index: " + fn
+
+
 def test_two_gpus_equal_one_gpu():
-    """SMR_GPUS=2 (one context and one worker thread per GPU, batches in flight concurrently) writes what SMR_GPUS=1 writes.
-    Needs two devices (gpurun --gpus 2); 2000-read batches so that both GPUs get several."""
+    """SMR_GPUS=2 (one context and one worker thread per GPU, batches in flight concurrently) writes what SMR_GPUS=1 writes, on
+    the stored sample of BASELINE config 4.  Needs two devices; 200-read batches so that both GPUs get several."""
     from sortmerna_b200 import api
+    if not os.path.exists(os.path.join(REF_DIR, "sortmerna_gpu")):
+        pytest.skip("oracle/_ref/sortmerna_gpu not built (oracle/Makefile.ref)")
     if api.load_library().smr_device_count() < 2:
         pytest.skip("needs two GPUs")
-    fastas, reads, idx = _config4_inputs()
     d = tempfile.mkdtemp(prefix="smr_2gpu_")
     try:
+        fastas, reads, idx = _config4_sample(d)
         extra = ["-sam", "-fastx", "-other", "-paired_in"]
-        one, _ = _run_binary("sortmerna_gpu", fastas, reads, idx, os.path.join(d, "g1"), extra, env=dict(os.environ, SMR_GPUS="1", SMR_BATCH_READS="2000"))
-        two, log = _run_binary("sortmerna_gpu", fastas, reads, idx, os.path.join(d, "g2"), extra, env=dict(os.environ, SMR_GPUS="2", SMR_BATCH_READS="2000"))
+        one, _ = _run_binary("sortmerna_gpu", fastas, reads, idx, os.path.join(d, "g1"), extra, env=dict(os.environ, SMR_GPUS="1", SMR_BATCH_READS="200"))
+        two, log = _run_binary("sortmerna_gpu", fastas, reads, idx, os.path.join(d, "g2"), extra, env=dict(os.environ, SMR_GPUS="2", SMR_BATCH_READS="200"))
         assert "resident on 2 GPU(s)" in log
         for fn in one:
             assert one[fn] == two[fn], fn

@@ -1,6 +1,9 @@
 """ora_ssw_align (the restated ssw_init + ssw_align, ssw.c:788-941) against the reference's OWN ssw.c,
-compiled unmodified into oracle/_ref/libssw_ref.so by oracle/Makefile.ref."""
+compiled unmodified into oracle/_ref/libssw_ref.so by oracle/Makefile.ref.  Where that library is absent, the reference's
+results come from tests/golden/ssw_reference.json, recorded from it by this file's __main__: a digest of every 100 cases."""
 import ctypes as C
+import hashlib
+import json
 import os
 
 import numpy as np
@@ -8,7 +11,9 @@ import pytest
 
 from oracle import ora
 
-pytestmark = pytest.mark.skipif(not os.path.exists(ora.REF_SSW), reason="oracle/_ref/libssw_ref.so not built")
+GOLDEN_REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ssw_reference.json")
+SCORES = [(2, -3, -3, 5, 2), (2, -4, -2, 6, 3), (1, -3, -3, 5, 2), (2, -7, -7, 3, 1)]
+BLOCK = 100
 
 
 class SAlign(C.Structure):  # s_align, include/ssw.h:58-71
@@ -46,28 +51,75 @@ def make_pair(rng, qlen, tlen, err, nfrac=0.0):
     return np.concatenate([flank, q]), t
 
 
-@pytest.mark.parametrize("scores", [(2, -3, -3, 5, 2), (2, -4, -2, 6, 3), (1, -3, -3, 5, 2), (2, -7, -7, 3, 1)])
-def test_ssw_restatement_matches_reference_ssw(scores):
+def reference_lib():
     lib = C.CDLL(ora.REF_SSW)
     lib.ssw_init.restype = C.c_void_p
     lib.ssw_init.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_int8]
     lib.ssw_align.restype = C.POINTER(SAlign)
     lib.ssw_align.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_uint8, C.c_uint8, C.c_uint8, C.c_uint16, C.c_int32, C.c_int32]
+    return lib
+
+
+def cases(scores):
+    """(q, t, filters) of the 1500 pairs of one scoring set"""
     match, mis, sn, go, ge = scores
-    mat = ora.score_matrix(match, mis, sn)
     rng = np.random.default_rng(1234 + match * 7 + go)
-    n_word = 0
     for it in range(1500):
         qlen = int(rng.integers(20, 181)) if it % 10 else int(rng.integers(250, 500))
         tlen = qlen + int(rng.integers(-10, 40))
         q, t = make_pair(rng, qlen, max(20, tlen), float(rng.choice([0.0, 0.01, 0.05, 0.15])), nfrac=0.01 if it % 7 == 0 else 0.0)
-        filters = int(rng.integers(0, 60))
-        exp = ref_ssw(lib, q, t, mat, go, ge, filters)
+        yield q, t, int(rng.integers(0, 60))
+
+
+def pinned(score, ref_begin, ref_end, read_begin, read_end, cigar, filters):
+    """what the comparison pins: score and end points always, begin points and CIGAR where the score passes the filter"""
+    return [score, ref_end, read_end] + ([ref_begin, read_begin, cigar] if score >= filters else [])
+
+
+def block_digests(rows):
+    return [hashlib.sha256(json.dumps(rows[k:k + BLOCK]).encode()).hexdigest()[:16] for k in range(0, len(rows), BLOCK)]
+
+
+def reference_results(scores):
+    """[pinned(...) per case], word-path count -- from the reference's ssw.c"""
+    lib = reference_lib()
+    match, mis, sn, go, ge = scores
+    mat = ora.score_matrix(match, mis, sn)
+    rows, n_word = [], 0
+    for q, t, filters in cases(scores):
+        e = ref_ssw(lib, q, t, mat, go, ge, filters)
+        rows.append(pinned(e[0], e[1], e[2], e[3], e[4], e[5], filters))
+        n_word += e[0] >= 255 - abs(min(mis, sn))
+    return rows, n_word
+
+
+@pytest.mark.parametrize("scores", SCORES)
+def test_ssw_restatement_matches_reference_ssw(scores):
+    match, mis, sn, go, ge = scores
+    mat = ora.score_matrix(match, mis, sn)
+    rows = []
+    for q, t, filters in cases(scores):
         rc, out, cig = ora.ssw_align(q, t, mat, go, ge, filters)
         assert rc == 0
-        assert int(out[0]) == exp[0] and int(out[2]) == exp[2] and int(out[4]) == exp[4], (it, out, exp[:5])
-        if exp[0] >= filters:
-            assert (int(out[1]), int(out[3])) == (exp[1], exp[3]), (it, out, exp[:5])
-            assert cig.tolist() == exp[5], (it, cig, exp[5])
-        n_word += exp[0] >= 255 - abs(min(mis, sn))
+        rows.append(pinned(int(out[0]), int(out[1]), int(out[2]), int(out[3]), int(out[4]), cig.tolist(), filters))
+    golden = json.load(open(GOLDEN_REF))[str(scores)]
+    if os.path.exists(ora.REF_SSW):
+        exp, n_word = reference_results(scores)
+        for it, (g, e) in enumerate(zip(rows, exp)):
+            assert g == e, (it, g, e)
+        assert {"blocks": block_digests(exp), "word_path_cases": int(n_word)} == golden    # the recording still describes the reference
+    else:
+        n_word = golden["word_path_cases"]
+        for k, (g, e) in enumerate(zip(block_digests(rows), golden["blocks"])):
+            assert g == e, f"cases {k * BLOCK}..{k * BLOCK + BLOCK - 1} differ from the reference's"
+        assert len(rows) == BLOCK * len(golden["blocks"])
     assert n_word > 20  # the int16 (word) path of the reference was exercised too
+
+
+if __name__ == "__main__":   # record tests/golden/ssw_reference.json from oracle/_ref/libssw_ref.so
+    rec = {}
+    for sc in SCORES:
+        exp, n_word = reference_results(sc)
+        rec[str(sc)] = {"blocks": block_digests(exp), "word_path_cases": int(n_word)}
+    with open(GOLDEN_REF, "w") as f:
+        json.dump(rec, f, indent=1)

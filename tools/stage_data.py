@@ -8,13 +8,14 @@ travels to the GPU box with the gpurun snapshot, like the built .so files):
                                       smr_build_index (our builder; tests/test_index_builder.py proves the files equal the
                                       reference builder's up to the arbitrary id numbering)
 
-`ensure_indexes()` is also what bench.py calls on the GPU box when data_cache/idx is incomplete
-(the FASTA files travel, the 1.1 GB of index files need not).
+`ensure_indexes()` is also what bench.py calls to index its databases in the temporary directory of a run
+(bench.py --db-dir data_cache/rRNA_databases measures against the staged databases).
 """
 import os
 import shutil
 import subprocess
 import sys
+import tempfile
 import time
 from concurrent.futures import ThreadPoolExecutor
 
@@ -73,9 +74,7 @@ def build_index_native(fasta, idx_dir, **kw):
 def build_index(fasta, idx_dir, extra=()):
     """Run the reference's index builder (indexdb.cpp:1119-2095) for one database (tests / cross-checks only)."""
     os.makedirs(idx_dir, exist_ok=True)
-    wd = os.path.join(CACHE, "_work", os.path.basename(fasta) + f".{os.getpid()}")
-    shutil.rmtree(wd, ignore_errors=True)
-    os.makedirs(wd)
+    wd = tempfile.mkdtemp(prefix="smr_idx_work_")
     tiny = os.path.join(wd, "tiny.fa")
     with open(tiny, "w") as f:
         f.write(">r\nACGTACGTACGTACGTACGTACGTACGTACGT\n")
