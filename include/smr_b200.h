@@ -239,6 +239,15 @@ int smr_debug_dpx_peak(smr_ctx*, double* giga_ops_per_s);
 int smr_debug_ssw(smr_ctx*, const uint8_t* q_cat, const uint64_t* q_off, const uint8_t* t_cat,
                   const uint64_t* t_off, uint32_t npairs, uint32_t filters, int32_t* out, uint32_t* cigars,
                   uint32_t cigar_cap);
+/* the candidate kernel's scorer path (fetcher staging + packed 16-bit pass or s32 fallback) on explicit tasks.
+ * q_cat: reads (codes 0..4, q_len bytes), t_cat: reference bytes (0..4, t_len bytes).  tasks[5*i..]: ref_abs, q_abs, n (window
+ * columns), m (query rows), minus -- minus = 1: q_abs names query element 0, read backwards and complemented.  pairs[2*k..]: task A,
+ * task B (0xFFFFFFFF: none).  One warp scores each run of `chain` consecutive pairs in order, as one scorer warp does (its query
+ * profile cache carries over).  scores[i]: the score published for task i; path[k]: 1 = packed pass, 0 = s32 fallback.
+ * SMR_ERR_ARG if a task reaches outside its buffer. */
+int smr_debug_sw_tasks(smr_ctx*, const uint8_t* q_cat, uint64_t q_len, const uint8_t* t_cat, uint64_t t_len,
+                       const uint32_t* tasks, uint32_t ntasks, const uint32_t* pairs, uint32_t npairs, uint32_t chain,
+                       uint32_t* scores, uint8_t* path);
 
 #ifdef __cplusplus
 }

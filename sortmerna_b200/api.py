@@ -27,7 +27,7 @@ SYMBOLS = ["smr_init", "smr_destroy", "smr_last_error", "smr_device_count", "smr
            "smr_run_resident", "smr_download_results", "smr_last_timings", "smr_debug_seed_windows", "smr_debug_ssw",
            "smr_debug_dpx_peak", "smr_set_stats_buffer", "smr_build_index", "smr_upload_fastx", "smr_resident_layout", "smr_pack_kvdb_blobs",
            "smr_set_aln_slots", "smr_aln_slots", "smr_aln_slots_needed", "smr_upload_fastx_gz", "smr_resident_text", "smr_debug_inflate",
-           "smr_build_index_device", "smr_debug_index_array", "smr_set_instrumentation"]
+           "smr_build_index_device", "smr_debug_index_array", "smr_set_instrumentation", "smr_debug_sw_tasks"]
 
 CNT_NAMES = ("num_aligned", "num_short", "sw_calls", "sw_cells", "windows", "trie_nodes", "buckets",
              "bucket_entries", "pos_entries", "lis_calls", "dbg_max_read_cycles", "dbg_sum_read_cycles", "dbg_lis_kernel_cycles",
@@ -392,6 +392,21 @@ class Aligner:
                                   C.c_uint32(filters), _ptr(out), _ptr(cig), C.c_uint32(cigar_cap))
         self._check(rc, "smr_debug_ssw")
         return out.reshape(n, 6), cig.reshape(n, cigar_cap)
+
+    def debug_sw_tasks(self, q_cat, t_cat, tasks, pairs, chain=1):
+        """The candidate kernel's scorer path on explicit tasks.  tasks: (ntasks, 5) rows (ref_abs, q_abs, n, m, minus) into t_cat /
+        q_cat (codes 0..4); pairs: (npairs, 2) task indices, -1 = no task B.  Returns (score per task, packed-path flag per pair)."""
+        q_cat = np.ascontiguousarray(q_cat, np.uint8)
+        t_cat = np.ascontiguousarray(t_cat, np.uint8)
+        tasks = np.ascontiguousarray(np.asarray(tasks, np.int64).reshape(-1, 5).astype(np.uint32))
+        pairs = np.ascontiguousarray(np.asarray(pairs, np.int64).reshape(-1, 2).astype(np.uint32))
+        scores = np.zeros(tasks.shape[0], np.uint32)
+        path = np.zeros(pairs.shape[0], np.uint8)
+        rc = self.L.smr_debug_sw_tasks(self.h, _ptr(q_cat), C.c_uint64(q_cat.size), _ptr(t_cat), C.c_uint64(t_cat.size), _ptr(tasks),
+                                       C.c_uint32(tasks.shape[0]), _ptr(pairs), C.c_uint32(pairs.shape[0]), C.c_uint32(chain),
+                                       _ptr(scores), _ptr(path))
+        self._check(rc, "smr_debug_sw_tasks")
+        return scores.astype(np.int64), path.astype(bool)
 
 
 def align_files(aligner: Aligner, batch: hostio.ReadBatch):

@@ -1350,4 +1350,52 @@ int smr_debug_ssw(smr_ctx* ctx, const uint8_t* q_cat, const uint64_t* q_off, con
   return SMR_OK;
 }
 
+int smr_debug_sw_tasks(smr_ctx* ctx, const uint8_t* q_cat, uint64_t q_len, const uint8_t* t_cat, uint64_t t_len, const uint32_t* tasks,
+                       uint32_t ntasks, const uint32_t* pairs, uint32_t npairs, uint32_t chain, uint32_t* scores, uint8_t* path) {
+  if (!ctx || !q_cat || !t_cat || (ntasks && (!tasks || !scores)) || (npairs && (!pairs || !path)) || chain == 0 || !ctx->have_params) return SMR_ERR_ARG;
+  if (ntasks >= kNoTask || q_len >= 0x80000000ull || t_len >= 0x80000000ull) return SMR_ERR_ARG;
+  std::vector<SwTask> tv(ntasks);
+  uint32_t row_cap = 1;
+  for (uint32_t i = 0; i < ntasks; ++i) {
+    const uint64_t ref = tasks[5 * i], qa = tasks[5 * i + 1], n = tasks[5 * i + 2], m = tasks[5 * i + 3], minus = tasks[5 * i + 4];
+    if (minus > 1 || ref + n > t_len) return SMR_ERR_ARG;
+    if (m == 0 ? qa > q_len : (minus ? qa >= q_len || qa + 1 < m : qa + m > q_len)) return SMR_ERR_ARG;   // minus strand: the query ends at q_abs
+    SwTask t{};
+    t.ref_abs = (uint32_t)ref; t.q_abs = (uint32_t)qa; t.alen = (uint32_t)n; t.qlen = (uint32_t)m; t.meta = (uint32_t)minus << 16;
+    tv[i] = t;
+    row_cap = std::max(row_cap, (uint32_t)n);
+  }
+  std::vector<uint32_t> pv(2 * (size_t)npairs);
+  for (uint32_t k = 0; k < npairs; ++k) {
+    const uint32_t a = pairs[2 * k], b = pairs[2 * k + 1];
+    if (a >= ntasks || (b != 0xFFFFFFFFu && b >= ntasks)) return SMR_ERR_ARG;
+    pv[2 * k] = a; pv[2 * k + 1] = b == 0xFFFFFFFFu ? kNoTask : b;
+  }
+  CK(cudaSetDevice(ctx->device));
+  const uint64_t nchains = ((uint64_t)npairs + chain - 1) / chain, ctas = std::max<uint64_t>(1, (nchains + kSwDebugWarps - 1) / kSwDebugWarps);
+  uint8_t *dq = nullptr, *dt = nullptr, *dpath = nullptr; SwTask* dtask = nullptr; uint32_t *dpairs = nullptr, *dscore = nullptr; int32_t* drows = nullptr;
+  // padded as the product pads its reads (seq04: +64 bytes) and references (refseq: +64 bytes of N), so that a window or query at the end
+  // of a buffer is staged exactly as in a run
+  CK(cudaMalloc(&dq, q_len + 64)); CK(cudaMalloc(&dt, t_len + 64));
+  CK(cudaMemset(dq + q_len, 0, 64)); CK(cudaMemset(dt + t_len, 4, 64));
+  if (q_len) CK(cudaMemcpy(dq, q_cat, q_len, cudaMemcpyHostToDevice));
+  if (t_len) CK(cudaMemcpy(dt, t_cat, t_len, cudaMemcpyHostToDevice));
+  CK(cudaMalloc(&dtask, (size_t)ntasks * sizeof(SwTask) + sizeof(SwTask))); CK(cudaMalloc(&dpairs, pv.size() * 4 + 8));
+  CK(cudaMalloc(&dscore, (size_t)ntasks * 4 + 4)); CK(cudaMalloc(&dpath, (size_t)npairs + 4));
+  CK(cudaMalloc(&drows, (size_t)ctas * kSwDebugWarps * 2 * row_cap * 4));
+  if (ntasks) CK(cudaMemcpy(dtask, tv.data(), (size_t)ntasks * sizeof(SwTask), cudaMemcpyHostToDevice));
+  if (npairs) CK(cudaMemcpy(dpairs, pv.data(), pv.size() * 4, cudaMemcpyHostToDevice));
+  CK(cudaMemset(dscore, 0xFF, (size_t)ntasks * 4 + 4)); CK(cudaMemset(dpath, 0xFF, (size_t)npairs + 4));   // a task no pair scores reads 0xFFFFFFFF
+  if (npairs) {
+    sw_tasks_debug_kernel<<<(unsigned)ctas, kSwDebugWarps * 32, kSwDebugWarps * kScorerSmem, ctx->stream>>>(dq, dt, dtask, dpairs, npairs, chain, to_dev(ctx->prm),
+                                                                                                          drows, row_cap, dscore, dpath);
+    CK(cudaGetLastError());
+  }
+  CK(cudaStreamSynchronize(ctx->stream));
+  if (ntasks) CK(cudaMemcpy(scores, dscore, (size_t)ntasks * 4, cudaMemcpyDeviceToHost));
+  if (npairs) CK(cudaMemcpy(path, dpath, npairs, cudaMemcpyDeviceToHost));
+  cudaFree(dq); cudaFree(dt); cudaFree(dtask); cudaFree(dpairs); cudaFree(dscore); cudaFree(dpath); cudaFree(drows);
+  return SMR_OK;
+}
+
 }  // extern "C"

@@ -1077,6 +1077,88 @@ __device__ void traverse_dev(PassEnv& E, ReadCtx& rc, const bool is_last_strand)
   } else if (ix.is_last && is_last_strand && rc.n_align > 0) rc.is_done = true;
 }
 
+// Stages one task pair into slot `sl` and arrives on its "full" mbarrier (ONE lane).  da / db: the first four words of the two
+// SwTask records (ref_abs, q_abs, alen, qlen), ma / mb their meta words; two = false: no task B.  Pairs the packed kernel cannot
+// score (sw_pair_ok) are marked slow and nothing is copied; an empty B task (no rows or no columns) rides along as a dead problem.
+// ref_of(meta) gives the reference buffer a task's window lies in; seq04: the reads.  Both must extend at least 15 bytes past the
+// last byte a task names (the copies are 16-byte aligned supersets).  The candidate kernel's fetcher and smr_debug_sw_tasks share it.
+template <class RefOf>
+__device__ __forceinline__ void stage_pair(ScSlot* sl, const uint4 da, const uint32_t ma, const bool two, const uint4 db, const uint32_t mb,
+                                           const uint8_t* const& seq04, const SwScore sc, const RefOf ref_of) {
+  const bool oka = da.w > 0 && da.z > 0 && sw_pair_ok((int32_t)da.w, (int32_t)da.z, sc);
+  const bool okb = !two || db.w == 0 || db.z == 0 || sw_pair_ok((int32_t)db.w, (int32_t)db.z, sc);
+  const bool fast = oka && okb;
+  const bool liveb = two && db.w > 0 && db.z > 0;
+  sl->slow = fast ? 0u : 1u;
+  sl->mA = da.w; sl->nA = da.z; sl->metaA = ma; sl->qabsA = da.y; sl->refA = da.x;
+  sl->mB = two ? db.w : 0u; sl->nB = two ? db.z : 0u; sl->metaB = mb; sl->qabsB = db.y; sl->refB = db.x;
+  if (!fast) mbar_arrive(&sl->bar);
+  else {
+    // 16-byte aligned supersets of [ref_abs, ref_abs + n) and of the query segment (minus strand: it ends at q_abs)
+    const uint8_t* ra = ref_of(ma);
+    const uint32_t wa0 = da.x & ~15u, wab = ((da.x & 15u) + da.z + 15u) & ~15u;
+    const uint32_t qsa = (ma & 0x10000u) ? da.y - (da.w - 1u) : da.y, qa0 = qsa & ~15u, qab = ((qsa & 15u) + da.w + 15u) & ~15u;
+    sl->woffA = kWinOff + (da.x & 15u); sl->qoffA = (ma & 0x10000u) ? (qsa & 15u) + da.w - 1u : (qsa & 15u);
+    uint32_t wb0 = 0, wbb = 0, qb0 = 0, qbb = 0; const uint8_t* rb = ra;
+    if (liveb) {
+      rb = ref_of(mb);
+      wb0 = db.x & ~15u; wbb = ((db.x & 15u) + db.z + 15u) & ~15u;
+      const uint32_t qsb = (mb & 0x10000u) ? db.y - (db.w - 1u) : db.y;
+      qb0 = qsb & ~15u; qbb = ((qsb & 15u) + db.w + 15u) & ~15u;
+      sl->woffB = kWinOff + (db.x & 15u); sl->qoffB = (mb & 0x10000u) ? (qsb & 15u) + db.w - 1u : (qsb & 15u);
+    } else { sl->woffB = kWinOff; sl->qoffB = 0; sl->mB = 0; sl->nB = 0; }
+    mbar_arrive_expect_tx(&sl->bar, wab + qab + wbb + qbb);
+    bulk_g2s(sl->win[0] + kWinOff, ra + wa0, wab, &sl->bar);
+    bulk_g2s(sl->q[0], seq04 + qa0, qab, &sl->bar);
+    if (liveb) { bulk_g2s(sl->win[1] + kWinOff, rb + wb0, wbb, &sl->bar); bulk_g2s(sl->q[1], seq04 + qb0, qbb, &sl->bar); }
+  }
+}
+
+// Scores the task pair staged in slot S (whole warp, after the slot's "full" mbarrier completed) into sa / sb; returns true when the
+// packed 16-bit pass ran, false for the s32 fallback.  s_prof: the two query profiles (kPairProfWords each), reused while keyq / keym
+// / keyR (the identity of the profile in each half: q_abs, qlen | rev << 31, and the R both were built for) say they still hold the
+// right query.  The fallback reads the inputs from global memory (ref_of, seq04) and scores a problem only if its window fits the row
+// scratch (rowH / rowF, row_cap ints each).  loaded(): called between profile set-up and the score pass; slow(): called when the
+// fallback ran (the instrumented kernel's phase clock and counters).  The candidate kernel's scorers and smr_debug_sw_tasks share it.
+// (Lazy arguments -- references, callbacks -- keep each global load inside the branch that needs it, as in the loop this came from.)
+template <class RefOf, class Loaded, class Slow>
+__device__ __forceinline__ bool score_slot(ScSlot& S, const bool two, uint32_t* s_prof, uint32_t (&keyq)[2], uint32_t (&keym)[2], int& keyR, const SwScore sc, const uint8_t* const& seq04,
+                                           const RefOf ref_of, int32_t* rowH, int32_t* rowF, const uint32_t& row_cap, const Loaded loaded,
+                                           const Slow slow, uint32_t& sa, uint32_t& sb) {
+  const int32_t mA = (int32_t)S.mA, nA = (int32_t)S.nA, mB = (int32_t)S.mB, nB = (int32_t)S.nB;
+  sa = 0; sb = 0;
+  if (!S.slow) {
+    const int R = pair_rows(max(mA, mB));
+    const int32_t nmax = max(nA, nB);
+    uint8_t* wa = S.win[0] + S.woffA; uint8_t* wb = S.win[1] + S.woffB;
+    pair_sentinels(wa, nA, nmax);
+    pair_sentinels(wb, nB, nmax);
+    const uint32_t kqa = S.qabsA, kma = (uint32_t)mA | ((S.metaA & 0x10000u) << 15), kqb = mB ? S.qabsB : 0xFFFFFFFEu, kmb = mB ? ((uint32_t)mB | ((S.metaB & 0x10000u) << 15)) : 0u;
+    // the two tasks of a pair are usually steps of one read on one strand with the same query segment: one profile serves both
+    if (R != keyR) { keyq[0] = keyq[1] = 0xFFFFFFFFu; keyR = R; }
+    if (!(keyq[0] == kqa && keym[0] == kma)) { const bool rev = (S.metaA & 0x10000u) != 0; pair_profile(S.q[0] + S.qoffA, rev ? -1 : 1, rev, mA, R, sc, s_prof); keyq[0] = kqa; keym[0] = kma; }
+    const uint32_t* profB = s_prof;
+    if (!(kqb == kqa && kmb == kma)) {
+      if (!(keyq[1] == kqb && keym[1] == kmb)) { const bool rev = (S.metaB & 0x10000u) != 0; pair_profile(S.q[1] + S.qoffB, rev ? -1 : 1, rev, mB, R, sc, s_prof + kPairProfWords); keyq[1] = kqb; keym[1] = kmb; }
+      profB = s_prof + kPairProfWords;
+    }
+    __syncwarp();
+    loaded();
+    const uint32_t r2 = sw_pair_dispatch(R, s_prof, profB, wa, wb, nmax, sc);
+    sa = r2 & 0xFFFFu; sb = r2 >> 16;
+    return true;
+  }
+  // shapes or scoring schemes outside the 16-bit kernel: the s32 wavefront (row blocks for long queries), from global memory
+  keyR = 0;
+  const bool reva = (S.metaA & 0x10000u) != 0, revb = (S.metaB & 0x10000u) != 0;
+  if (mA > 0 && nA > 0 && (uint32_t)nA <= row_cap)
+    sa = (uint32_t)sw_forward_any(SeqView{seq04, (int32_t)S.qabsA, reva ? -1 : 1, reva}, mA, SeqView{ref_of(S.metaA), (int32_t)S.refA, 1, false}, nA, sc, rowH, rowF).score;
+  if (two && mB > 0 && nB > 0 && (uint32_t)nB <= row_cap)
+    sb = (uint32_t)sw_forward_any(SeqView{seq04, (int32_t)S.qabsB, revb ? -1 : 1, revb}, mB, SeqView{ref_of(S.metaB), (int32_t)S.refB, 1, false}, nB, sc, rowH, rowF).score;
+  slow();
+  return false;
+}
+
 // ---- fetcher role: one lane per (scorer, slot) pops task pairs from the queue and stages their inputs ----
 __device__ void fetcher_loop(const DevBatch& b, const DevParams& prm, const LisGlobals& g, uint8_t* scorer_smem) {
   const unsigned lane = lane_id();
@@ -1108,33 +1190,7 @@ __device__ void fetcher_loop(const DevBatch& b, const DevParams& prm, const LisG
             const bool two = tb != kNoTask;
             uint4 db = make_uint4(0, 0, 0, 0); uint32_t mb = 0;
             if (two) { db = __ldcg((const uint4*)(tasks + tb)); mb = __ldcg(&tasks[tb].meta); }
-            const bool oka = da.w > 0 && da.z > 0 && sw_pair_ok((int32_t)da.w, (int32_t)da.z, sc);
-            const bool okb = !two || db.w == 0 || db.z == 0 || sw_pair_ok((int32_t)db.w, (int32_t)db.z, sc);
-            const bool fast = oka && okb;
-            const bool liveb = two && db.w > 0 && db.z > 0;
-            sl->slow = fast ? 0u : 1u;
-            sl->mA = da.w; sl->nA = da.z; sl->metaA = ma; sl->qabsA = da.y; sl->refA = da.x;
-            sl->mB = two ? db.w : 0u; sl->nB = two ? db.z : 0u; sl->metaB = mb; sl->qabsB = db.y; sl->refB = db.x;
-            if (!fast) mbar_arrive(&sl->bar);
-            else {
-              // 16-byte aligned supersets of [ref_abs, ref_abs + n) and of the query segment (minus strand: it ends at q_abs)
-              const uint8_t* ra = g.parts[ma & 0xFFFFu].refseq;
-              const uint32_t wa0 = da.x & ~15u, wab = ((da.x & 15u) + da.z + 15u) & ~15u;
-              const uint32_t qsa = (ma & 0x10000u) ? da.y - (da.w - 1u) : da.y, qa0 = qsa & ~15u, qab = ((qsa & 15u) + da.w + 15u) & ~15u;
-              sl->woffA = kWinOff + (da.x & 15u); sl->qoffA = (ma & 0x10000u) ? (qsa & 15u) + da.w - 1u : (qsa & 15u);
-              uint32_t wb0 = 0, wbb = 0, qb0 = 0, qbb = 0; const uint8_t* rb = ra;
-              if (liveb) {
-                rb = g.parts[mb & 0xFFFFu].refseq;
-                wb0 = db.x & ~15u; wbb = ((db.x & 15u) + db.z + 15u) & ~15u;
-                const uint32_t qsb = (mb & 0x10000u) ? db.y - (db.w - 1u) : db.y;
-                qb0 = qsb & ~15u; qbb = ((qsb & 15u) + db.w + 15u) & ~15u;
-                sl->woffB = kWinOff + (db.x & 15u); sl->qoffB = (mb & 0x10000u) ? (qsb & 15u) + db.w - 1u : (qsb & 15u);
-              } else { sl->woffB = kWinOff; sl->qoffB = 0; sl->mB = 0; sl->nB = 0; }
-              mbar_arrive_expect_tx(&sl->bar, wab + qab + wbb + qbb);
-              bulk_g2s(sl->win[0] + kWinOff, ra + wa0, wab, &sl->bar);
-              bulk_g2s(sl->q[0], b.seq04 + qa0, qab, &sl->bar);
-              if (liveb) { bulk_g2s(sl->win[1] + kWinOff, rb + wb0, wbb, &sl->bar); bulk_g2s(sl->q[1], b.seq04 + qb0, qbb, &sl->bar); }
-            }
+            stage_pair(sl, da, ma, two, db, mb, b.seq04, sc, [&](const uint32_t& meta) { return g.parts[meta & 0xFFFFu].refseq; });
           }
         }
       }
@@ -1176,36 +1232,9 @@ __device__ void scorer_loop(const DevBatch& b, const DevParams& prm, const LisGl
     const uint32_t ta = S.ta, tb = S.tb;
     const bool two = tb != kNoTask;
     const int32_t mA = (int32_t)S.mA, nA = (int32_t)S.nA, mB = (int32_t)S.mB, nB = (int32_t)S.nB;
-    uint32_t sa = 0, sb = 0;
-    if (!S.slow) {
-      const int R = pair_rows(max(mA, mB));
-      const int32_t nmax = max(nA, nB);
-      uint8_t* wa = S.win[0] + S.woffA; uint8_t* wb = S.win[1] + S.woffB;
-      pair_sentinels(wa, nA, nmax);
-      pair_sentinels(wb, nB, nmax);
-      const uint32_t kqa = S.qabsA, kma = (uint32_t)mA | ((S.metaA & 0x10000u) << 15), kqb = mB ? S.qabsB : 0xFFFFFFFEu, kmb = mB ? ((uint32_t)mB | ((S.metaB & 0x10000u) << 15)) : 0u;
-      // the two tasks of a pair are usually steps of one read on one strand with the same query segment: one profile serves both
-      if (R != keyR) { keyq[0] = keyq[1] = 0xFFFFFFFFu; keyR = R; }
-      if (!(keyq[0] == kqa && keym[0] == kma)) { const bool rev = (S.metaA & 0x10000u) != 0; pair_profile(S.q[0] + S.qoffA, rev ? -1 : 1, rev, mA, R, sc, s_prof); keyq[0] = kqa; keym[0] = kma; }
-      const uint32_t* profB = s_prof;
-      if (!(kqb == kqa && kmb == kma)) {
-        if (!(keyq[1] == kqb && keym[1] == kmb)) { const bool rev = (S.metaB & 0x10000u) != 0; pair_profile(S.q[1] + S.qoffB, rev ? -1 : 1, rev, mB, R, sc, s_prof + kPairProfWords); keyq[1] = kqb; keym[1] = kmb; }
-        profB = s_prof + kPairProfWords;
-      }
-      __syncwarp();
-      { const long long t2 = lis_clock<kInstr>(); cy_load += (unsigned long long)(t2 - tq); tq = t2; }
-      const uint32_t r2 = sw_pair_dispatch(R, s_prof, profB, wa, wb, nmax, sc);
-      sa = r2 & 0xFFFFu; sb = r2 >> 16;
-    } else {
-      // shapes or scoring schemes outside the 16-bit kernel: the s32 wavefront (row blocks for long queries), from global memory
-      keyR = 0;
-      const bool reva = (S.metaA & 0x10000u) != 0, revb = (S.metaB & 0x10000u) != 0;
-      if (mA > 0 && nA > 0 && (uint32_t)nA <= g.row_cap)
-        sa = (uint32_t)sw_forward_any(SeqView{b.seq04, (int32_t)S.qabsA, reva ? -1 : 1, reva}, mA, SeqView{g.parts[S.metaA & 0xFFFFu].refseq, (int32_t)S.refA, 1, false}, nA, sc, rowH, rowF).score;
-      if (two && mB > 0 && nB > 0 && (uint32_t)nB <= g.row_cap)
-        sb = (uint32_t)sw_forward_any(SeqView{b.seq04, (int32_t)S.qabsB, revb ? -1 : 1, revb}, mB, SeqView{g.parts[S.metaB & 0xFFFFu].refseq, (int32_t)S.refB, 1, false}, nB, sc, rowH, rowF).score;
-      ++n_slow;
-    }
+    uint32_t sa, sb;
+    score_slot(S, two, s_prof, keyq, keym, keyR, sc, b.seq04, [&](const uint32_t& meta) { return g.parts[meta & 0xFFFFu].refseq; }, rowH, rowF, g.row_cap,
+               [&] { const long long t2 = lis_clock<kInstr>(); cy_load += (unsigned long long)(t2 - tq); tq = t2; }, [&] { ++n_slow; }, sa, sb);
     ++n_pairs; n_cells += (unsigned long long)nA * mA + (unsigned long long)nB * mB;
     if (SMR_EXP_SCORER_DELAY) exp_delay(tq, SMR_EXP_SCORER_DELAY);
     { const long long t2 = lis_clock<kInstr>(); cy_sw += (unsigned long long)(t2 - tq); tq = t2; }
@@ -1364,6 +1393,56 @@ lis_kernel(DevBatch b, DevParams prm, LisGlobals g) {
         }
       }
     }
+  }
+}
+
+// unit-test kernel (smr_debug_sw_tasks): the scorer path of the candidate kernel on explicit task pairs.  One warp per chain of
+// `chain` consecutive pairs, scored in order with one profile cache and the two input slots taken in turn, as one scorer warp does;
+// lane 0 stages each pair as the fetcher does.  tasks: ref_abs into tcat, q_abs into qcat, meta = minus strand << 16.
+// pairs[2k], pairs[2k + 1]: the task indices of pair k (B = kNoTask: none).  scores[t]: what the scorer publishes for task t;
+// path[k]: 1 = packed 16-bit pass, 0 = s32 fallback.  rows: 2 * row_cap ints of fallback scratch per warp.
+constexpr int kSwDebugWarps = 4;
+__global__ void __launch_bounds__(kSwDebugWarps * 32)
+sw_tasks_debug_kernel(const uint8_t* qcat, const uint8_t* tcat, const SwTask* tasks, const uint32_t* pairs, uint32_t npairs, uint32_t chain,
+                      DevParams prm, int32_t* rows, uint32_t row_cap, uint32_t* scores, uint8_t* path) {
+  extern __shared__ __align__(16) uint8_t dbg_smem[];   // kSwDebugWarps * kScorerSmem: the scorer layout, profiles then slots
+  const unsigned lane = lane_id();
+  const uint32_t w = threadIdx.x >> 5, warp = blockIdx.x * kSwDebugWarps + w;
+  uint8_t* sm = dbg_smem + (size_t)w * kScorerSmem;
+  uint32_t* s_prof = (uint32_t*)sm;
+  ScSlot* slots = (ScSlot*)(sm + 2 * kPairProfWords * 4);
+  if (lane < 2u) mbar_init(&slots[lane].bar, 1);
+  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  __syncwarp();
+  const SwScore sc{prm.match, prm.mismatch, prm.score_N, prm.gap_open, prm.gap_ext, prm.one};
+  int32_t* rowH = rows + (size_t)warp * 2 * row_cap; int32_t* rowF = rowH + row_cap;
+  const auto ref_of = [&](const uint32_t&) { return tcat; };
+  // identity of the query profile resident in each half: (q_abs, qlen | rev << 31, R)
+  uint32_t keyq[2] = {0xFFFFFFFFu, 0xFFFFFFFFu}, keym[2] = {0xFFFFFFFFu, 0xFFFFFFFFu}; int keyR = 0;
+  uint32_t par[2] = {0, 0};
+  const uint64_t k0 = (uint64_t)warp * chain, k1 = min(k0 + chain, (uint64_t)npairs);
+  for (uint64_t k = k0; k < k1; ++k) {
+    const int s = (int)((k - k0) & 1u);
+    ScSlot* sl = slots + s;
+    const uint32_t ta = pairs[2 * k], tb = pairs[2 * k + 1];
+    const bool two = tb != kNoTask;
+    // the slot's previous pair was read (and its sentinels written) through the generic proxy; the bulk copies write through the async one
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    __syncwarp();
+    if (lane == 0) {
+      const uint4 da = *(const uint4*)(tasks + ta);
+      const uint32_t ma = tasks[ta].meta;
+      uint4 db = make_uint4(0, 0, 0, 0); uint32_t mb = 0;
+      if (two) { db = *(const uint4*)(tasks + tb); mb = tasks[tb].meta; }
+      sl->planner = 0; sl->ta = ta; sl->tb = tb;
+      stage_pair(sl, da, ma, two, db, mb, qcat, sc, ref_of);
+    }
+    while (!mbar_try_wait(&sl->bar, par[s])) {}
+    par[s] ^= 1u;
+    uint32_t sa, sb;
+    const bool packed = score_slot(*sl, two, s_prof, keyq, keym, keyR, sc, qcat, ref_of, rowH, rowF, row_cap, [] {}, [] {}, sa, sb);
+    __syncwarp();
+    if (lane == 0) { scores[ta] = sa; if (two) scores[tb] = sb; path[k] = packed ? 1 : 0; }
   }
 }
 

@@ -93,6 +93,23 @@ def test_ssw_matches_oracle(aligner, scores):
             q[int(rng.integers(0, q.size))] = 4
             t[int(rng.integers(0, t.size))] = 4
         qs.append(q); ts.append(t)
+    # queries shorter than 18, windows of 193..449 columns (both staged-window widths and the 448-column stage limit of the
+    # score-only kernels) and windows shorter than the query
+    rng2 = np.random.default_rng(199)
+    for it in range(300):
+        kind = it % 3
+        qlen = int(rng2.integers(1, 18)) if kind == 0 else int(rng2.integers(18, 257))
+        tlen = int(rng2.integers(193, 450)) if kind < 2 else int(rng2.integers(1, qlen + 1))
+        q = rng2.integers(0, 4, qlen).astype(np.uint8)
+        t = rng2.integers(0, 4, tlen).astype(np.uint8)
+        k = min(qlen, tlen)
+        p, o = int(rng2.integers(0, tlen - k + 1)), int(rng2.integers(0, qlen - k + 1))
+        t[p:p + k] = q[o:o + k]
+        m = rng2.random(tlen) < float(rng2.choice([0.0, 0.02, 0.1]))
+        t[m] = rng2.integers(0, 4, int(m.sum()))
+        if it % 7 == 0:
+            q[int(rng2.integers(0, qlen))] = 4
+        qs.append(q); ts.append(t)
     q_off = np.zeros(len(qs) + 1, np.uint64); np.cumsum([x.size for x in qs], out=q_off[1:])
     t_off = np.zeros(len(ts) + 1, np.uint64); np.cumsum([x.size for x in ts], out=t_off[1:])
     out, cig = aligner.debug_ssw(np.concatenate(qs), q_off, np.concatenate(ts), t_off, filters=30, cigar_cap=512)

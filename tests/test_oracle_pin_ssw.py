@@ -12,7 +12,9 @@ import pytest
 from oracle import ora
 
 GOLDEN_REF = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ssw_reference.json")
-SCORES = [(2, -3, -3, 5, 2), (2, -4, -2, 6, 3), (1, -3, -3, 5, 2), (2, -7, -7, 3, 1)]
+SCORES = [(2, -3, -3, 5, 2), (2, -4, -2, 6, 3), (1, -3, -3, 5, 2), (2, -7, -7, 3, 1),
+          # the schemes tests/test_gpu_sw_scorer.py adds: gap_ext == gap_open, gap_ext == 0, score_N = 0, and the edges of the int8 matrix
+          (2, -3, -3, 4, 4), (2, -3, -3, 5, 0), (2, -3, 0, 5, 2), (125, -128, -128, 255, 1), (126, -128, -128, 255, 1)]
 BLOCK = 100
 
 
@@ -64,8 +66,12 @@ def cases(scores):
     """(q, t, filters) of the 1500 pairs of one scoring set"""
     match, mis, sn, go, ge = scores
     rng = np.random.default_rng(1234 + match * 7 + go)
+    # the reference's word kernel saturates at 32767 (ssw.c:399-575) where the restatement keeps counting: with large match scores the
+    # queries stay short enough (flank included) that no score gets there
+    qmax = 32767 // match - 8
     for it in range(1500):
         qlen = int(rng.integers(20, 181)) if it % 10 else int(rng.integers(250, 500))
+        qlen = min(qlen, qmax)
         tlen = qlen + int(rng.integers(-10, 40))
         q, t = make_pair(rng, qlen, max(20, tlen), float(rng.choice([0.0, 0.01, 0.05, 0.15])), nfrac=0.01 if it % 7 == 0 else 0.0)
         yield q, t, int(rng.integers(0, 60))
